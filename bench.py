@@ -49,7 +49,43 @@ def parse_args():
     ap.add_argument("--results-csv", default=None, help="also merge this run into a CSV with the reference bench tool's schema and codec naming (pcodec_b200/benchfmt.py)")
     ap.add_argument("--no-gather-pages", action="store_true", help="N > 1: exchange only the per-chunk sizes; the default also gathers the compressed pages on the device (every rank ends up with the whole file)")
     ap.add_argument("--gather-ctas", type=int, default=0, help="CTAs of the page-gather copy kernel (it runs beside the next step's kernels on a high-priority stream); 0 = 16 per rank of the job, at most 64 (profiles/r02_zz3_gather_sweep.txt)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned to its caller (rank 0) as DIR/<name>.npy: seeded samples of the decompressed "
+                         "numbers (float64), of the compressed file and of its side index (bytes as float32), and every chunk's compressed size (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs the GPU arm (--impl ours)")
+    return args
+
+
+# Sizes of the --dump-outputs samples: 16 + 16 + 4 MiB as written, under 64 MiB with the per-chunk sizes.  Positions come from
+# DUMP_SEED and the array's length alone, so two builds that return the same outputs write the same files.
+DUMP_SEED = 20251017
+DUMP_NUMS, DUMP_FILE_BYTES, DUMP_INDEX_BYTES = 1 << 21, 1 << 22, 1 << 20
+
+
+def dump_positions(length, k):
+    """Sorted positions of the dump's sample of an array of `length` elements: all of them when there are at most `k`."""
+    if length <= k:
+        return np.arange(length, dtype=np.int64)
+    return np.sort(np.random.default_rng([DUMP_SEED, length]).integers(0, length, size=k, dtype=np.int64))
+
+
+def dump_outputs(out_dir, d_out, d_comp, n_comp, d_index, n_index, chunk_offs):
+    """Writes the last timed step's outputs.  The numbers of this workload stay below 2^53, so float64 holds them exactly."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+
+    def sample(t, length, k):
+        return t[torch.from_numpy(dump_positions(length, k)).to(t.device)].cpu()
+
+    np.save(os.path.join(out_dir, "decompressed.npy"), sample(d_out, d_out.numel(), DUMP_NUMS).numpy().view(np.uint64).astype(np.float64))
+    np.save(os.path.join(out_dir, "compressed.npy"), sample(d_comp, n_comp, DUMP_FILE_BYTES).numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "index.npy"), sample(d_index, n_index, DUMP_INDEX_BYTES).numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "chunk_compressed_bytes.npy"), np.diff(np.asarray(chunk_offs, dtype=np.float64)))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -410,10 +446,14 @@ def run_gpu_arm(args, rank, world):
     # chunk c in the GPU's file must be the oracle's chunk bytes for the same numbers and ChunkConfig
     import struct
 
-    ih = bytes(d_index[:64].cpu().numpy())
-    n_idx_chunks, chunks_off = struct.unpack_from("<Q", ih, 8)[0], struct.unpack_from("<Q", ih, 32)[0]
-    recs = bytes(d_index[chunks_off:chunks_off + 32 * n_idx_chunks].cpu().numpy())
-    chunk_offs = [struct.unpack_from("<Q", recs, 32 * i)[0] for i in range(n_idx_chunks)] + [Cbytes - 1]  # the terminator byte ends the file
+    def index_chunks(d_index, file_len):
+        """(chunk count, the index's 32-byte chunk records, every chunk's start offset in the file followed by the terminator's)."""
+        ih = bytes(d_index[:64].cpu().numpy())
+        n_idx_chunks, chunks_off = struct.unpack_from("<Q", ih, 8)[0], struct.unpack_from("<Q", ih, 32)[0]
+        recs = bytes(d_index[chunks_off:chunks_off + 32 * n_idx_chunks].cpu().numpy())
+        return n_idx_chunks, recs, [struct.unpack_from("<Q", recs, 32 * i)[0] for i in range(n_idx_chunks)] + [file_len - 1]  # the terminator byte ends the file
+
+    n_idx_chunks, recs, chunk_offs = index_chunks(d_index, Cbytes)
     parity = {"checked_chunks": 0, "against": "oracle/ (C++ restatement of pco 1.0.3), same numbers and ChunkConfig"}
     try:
         from oracle import pyoracle
@@ -468,6 +508,8 @@ def run_gpu_arm(args, rank, world):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t.item())
     ms_per_step = total_ms / max(args.steps, 1)
+    if args.dump_outputs and rank == 0:  # before the index-free leg below decodes into d_out again
+        dump_outputs(args.dump_outputs, d_out, d_comp, n_written.value, d_index, ilen.value, index_chunks(d_index, n_written.value)[2])
     if gather_on and gather_info is not None:
         gather_info["device_ms"] = float(np.mean([a.elapsed_time(b) for a, b in gather_events])) if gather_events else None
         gather_info["ctas"] = gather_ctas

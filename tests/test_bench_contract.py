@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -19,3 +21,10 @@ def test_reference_arm_prints_one_contract_line():
         assert key in d, key
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_refuses_arguments_it_cannot_honour(argv, tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120, cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr, out.stderr[-2000:]
+    assert not out.stdout.strip() and not os.listdir(tmp_path)
