@@ -89,6 +89,32 @@ PcoB200Error pco_b200_decompress_ex(const void *compressed, size_t compressed_le
                                     size_t dst_len, PcoB200Progress *progress, const void *index, size_t index_len,
                                     uint32_t flags, void *cuda_stream);
 
+/* Stream-ordered decompress of a file whose bytes, side index and destination all live in device memory (no reference
+ * counterpart).  The call only enqueues work on `cuda_stream`: no device-to-host copy, no synchronisation, no allocation, so a
+ * caller can keep issuing work on the same thread and can capture the call in a CUDA graph.  The caller declares n_chunks and
+ * n_total (what the compress that wrote the index reported) and passes a workspace of at least
+ * pco_b200_decompress_async_workspace_size(n_total, n_chunks, dtype) bytes that no other call uses while this one runs.
+ * The return value only reports the arguments: PCO_B200_INVALID_TYPE for an unknown dtype, PCO_B200_INVALID_ARGUMENT for a null
+ * pointer, n_chunks == 0, dst_len < n_total, an index shorter than its chunk table or not 8-byte aligned, or a workspace that is
+ * too small; PCO_B200_CUDA without a device or for a launch failure.  What the device finds lands in *d_result (device memory)
+ * when the stream reaches it: `status` is the PcoB200Error pco_b200_decompress_ex returns for the same bytes, `first_bad_chunk`
+ * the lowest failing chunk (0xffffffff when the file header or the side index failed, or nothing did).  Files the fast kernels
+ * decline (Dict, Lookback, Conv1, tANS tables over 2^10 states) report PCO_B200_UNSUPPORTED: this path has no cold fallback.
+ * The first call on a thread (and on a device) does one-time set-up that cannot be captured; call
+ * pco_b200_decompress_async_prepare(dtype) before capturing. */
+typedef struct PcoB200AsyncResult {
+  uint32_t status;          /* PcoB200Error */
+  uint32_t first_bad_chunk;
+  uint64_t n_total;         /* numbers the file holds (= numbers written when status is PCO_B200_OK) */
+  uint32_t finished;        /* 1: the whole file was decoded (pco::Progress::finished) */
+  uint32_t reserved;
+} PcoB200AsyncResult;
+size_t pco_b200_decompress_async_workspace_size(size_t n_total, size_t n_chunks, unsigned char dtype);
+PcoB200Error pco_b200_decompress_async_prepare(unsigned char dtype);
+PcoB200Error pco_b200_decompress_async(const void *d_src, size_t src_len, unsigned char dtype, const void *d_index, size_t index_len,
+                                       size_t n_chunks, size_t n_total, void *d_dst, size_t dst_len, void *d_workspace,
+                                       size_t workspace_len, PcoB200AsyncResult *d_result, void *cuda_stream);
+
 /* pco::standalone::simple_compress (pco/src/standalone/simple.rs:58-91): header carries uniform type 0.
  * config may be NULL (pco::ChunkConfig::default()).  Fails with PCO_B200_IO if dst is too small. */
 PcoB200Error pco_b200_simple_compress(const void *nums, size_t n, unsigned char dtype, const PcoB200ChunkConfig *config,

@@ -474,7 +474,9 @@ __device__ __forceinline__ void fused_decoder(FusedSmem& sm, const FileParams& f
 template <typename L>
 __global__ void __launch_bounds__(FZ_THREADS, PCOB_FZ_MIN_BLOCKS)
 fused_narrow_kernel(FileParams fp, const IndexChunk* __restrict__ chunks, const uint8_t* __restrict__ index_base, uint64_t index_len,
-                    uint32_t* __restrict__ statuses, uint8_t* __restrict__ d_cls, L* __restrict__ out, uint64_t out_len) {
+                    uint32_t* __restrict__ statuses, uint8_t* __restrict__ d_cls, L* __restrict__ out, uint64_t out_len,
+                    const uint32_t* __restrict__ gate) {
+  if (gate_closed(gate, fp)) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   FusedSmem& sm = *reinterpret_cast<FusedSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;

@@ -226,6 +226,27 @@ struct FileParams {
   uint32_t format_major;
 };
 
+// Stream-ordered decompress (pco_b200_decompress_async, decode_async.cuh) parses the standalone header and checks the side index on
+// the device: async_validate_kernel leaves an AsyncGate in the caller's workspace, and the decode kernels read it in their prologue
+// as `const uint32_t* gate`.  A closed gate makes every CTA return at once; an open one carries the header fields the host would
+// otherwise have put into FileParams.  gate == nullptr on every other entry point (the host parsed the header).
+struct AsyncGate {
+  uint32_t open;          // 1: header and index passed; 0: async_validate_kernel has written the result already
+  uint32_t uniform_type;  // from the standalone header
+  uint32_t format_major;
+  uint32_t finished;      // the index saw the file's terminator
+  uint64_t n_total;
+  uint64_t reserved;
+};
+__device__ __forceinline__ bool gate_closed(const uint32_t* gate, FileParams& fp) {
+  if (gate == nullptr) return false;
+  const AsyncGate* g = reinterpret_cast<const AsyncGate*>(gate);
+  if (g->open == 0) return true;
+  fp.uniform_type = g->uniform_type;
+  fp.format_major = g->format_major;
+  return false;
+}
+
 // ---------------------------------------------------------------------------
 // walk_kernel (K6): builds the side index of a standalone file in place.
 //   serial_file_mode = 1: a single CTA walks the file chunk after chunk from `first_chunk_byte`
@@ -907,7 +928,9 @@ struct SymWalkSmem {
 
 __global__ void __launch_bounds__(SW_THREADS) symwalk_kernel(FileParams fp, const IndexChunk* __restrict__ chunks, const uint8_t* __restrict__ index_base,
                                                               uint64_t index_len, uint64_t out_len, uint8_t* __restrict__ d_syms, uint32_t* __restrict__ d_offs,
-                                                              uint8_t* __restrict__ d_nvars, NarrowInfo* __restrict__ d_narrow, int classes_preset) {
+                                                              uint8_t* __restrict__ d_nvars, NarrowInfo* __restrict__ d_narrow, int classes_preset,
+                                                              const uint32_t* __restrict__ gate) {
+  if (gate_closed(gate, fp)) return;
   if (classes_preset && (d_nvars[blockIdx.x] & CLS_DONE)) return;  // fused_narrow_kernel has decoded (or refused) this chunk
   extern __shared__ __align__(16) unsigned char smem_raw[];
   SymWalkSmem& sm = *reinterpret_cast<SymWalkSmem*>(smem_raw);
@@ -1116,7 +1139,8 @@ template <typename L, int NV>
 __global__ void __launch_bounds__(DEC_THREADS, NV == 1 ? PCOB_DEC_NV1_BLOCKS : 2)
 decode_kernel(FileParams fp, const IndexChunk* __restrict__ chunks, uint32_t* __restrict__ statuses, const uint8_t* __restrict__ index_base, uint64_t index_len,
               L* __restrict__ out, uint64_t out_len, const Binoms* __restrict__ binoms, const uint8_t* __restrict__ d_syms,
-              const uint32_t* __restrict__ d_offs, const uint8_t* __restrict__ d_nvars) {
+              const uint32_t* __restrict__ d_offs, const uint8_t* __restrict__ d_nvars, const uint32_t* __restrict__ gate) {
+  if (gate_closed(gate, fp)) return;
   if (d_nvars[blockIdx.x] != NV) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   DecodeSmem& sm = *reinterpret_cast<DecodeSmem*>(smem_raw);

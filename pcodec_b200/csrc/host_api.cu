@@ -9,6 +9,7 @@
 #include "decode_fused.cuh"
 #include "gather_kernels.cuh"
 #include "decode_cold.cuh"
+#include "decode_async.cuh"
 #include "host_common.hpp"
 
 namespace pcob200 {
@@ -117,6 +118,23 @@ static auto dispatch_latent(uint32_t dtype, Fn&& fn) {
   }
 }
 
+// Function attributes of the decode kernels, set once per thread context (the first decode launch, or pco_b200_decompress_async_prepare).
+static PcoB200Error set_decode_attrs(Context& c) {
+  if (c.attrs_set) return PCO_B200_OK;
+  c.attrs_set = true;
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(symwalk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SymWalkSmem)));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(symwalk_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint16_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint8_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  return PCO_B200_OK;
+}
+
 struct DecodeOutcome {
   uint64_t n_total = 0;   // numbers in the chunks seen
   bool terminated = false;
@@ -145,19 +163,7 @@ static PcoB200Error launch_decode(Context& c, const FileParams& fp, const uint8_
   const IndexChunk* d_chunks = reinterpret_cast<const IndexChunk*>(d_index + chunks_offset);
   static const bool use_fused = [] { const char* e = std::getenv("PCOB200_FUSED"); return !(e && e[0] == '0'); }();
   const bool narrow_ok = true;  // the fused kernel serves every number width
-  if (!c.attrs_set) {
-    c.attrs_set = true;
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(symwalk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SymWalkSmem)));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(symwalk_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FusedSmem)));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint16_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    PCOB_CUDA_TRY(cudaFuncSetAttribute(fused_narrow_kernel<uint8_t>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-  }
+  if (PcoB200Error e = set_decode_attrs(c)) return e;
   c.last_decode_chunks = n_chunks;
   const uint32_t* st = static_cast<const uint32_t*>(c.pinned_res);
   bool fused_ran = false;
@@ -167,7 +173,7 @@ static PcoB200Error launch_decode(Context& c, const FileParams& fp, const uint8_
     profiler().begin("fused_narrow_kernel", stream);
     dispatch_latent(fp.dtype, [&](auto tag) {
       using L = decltype(tag);
-      fused_narrow_kernel<L><<<n_chunks, FZ_THREADS, sizeof(FusedSmem), stream>>>(fp, d_chunks, d_index, index_len, d_st, d_cls, static_cast<L*>(d_out), out_len);
+      fused_narrow_kernel<L><<<n_chunks, FZ_THREADS, sizeof(FusedSmem), stream>>>(fp, d_chunks, d_index, index_len, d_st, d_cls, static_cast<L*>(d_out), out_len, nullptr);
       return 0;
     });
     profiler().end(stream);
@@ -193,7 +199,7 @@ static PcoB200Error launch_decode(Context& c, const FileParams& fp, const uint8_
   if (old_narrow) PCOB_CUDA_TRY(c.dec_narrow.reserve(size_t(n_chunks) * sizeof(NarrowInfo)));
   profiler().begin("symwalk_kernel", stream);
   symwalk_kernel<<<n_chunks, SW_THREADS, sizeof(SymWalkSmem), stream>>>(fp, d_chunks, d_index, index_len, out_len, c.dec_syms.as<uint8_t>(), c.dec_offs.as<uint32_t>(),
-                                                                        d_cls, old_narrow ? c.dec_narrow.as<NarrowInfo>() : nullptr, fused_ran ? 1 : 0);
+                                                                        d_cls, old_narrow ? c.dec_narrow.as<NarrowInfo>() : nullptr, fused_ran ? 1 : 0, nullptr);
   profiler().end(stream);
   profiler().begin("decode_kernel", stream);  // the span covers every decode instantiation (a chunk runs in exactly one)
   if (old_narrow) {
@@ -207,9 +213,9 @@ static PcoB200Error launch_decode(Context& c, const FileParams& fp, const uint8_
   dispatch_latent(fp.dtype, [&](auto tag) {
     using L = decltype(tag);
     decode_kernel<L, 1><<<n_chunks, DEC_THREADS, sizeof(DecodeSmem), stream>>>(fp, d_chunks, d_st, d_index, index_len, static_cast<L*>(d_out), out_len, c.d_binoms,
-                                                                                c.dec_syms.as<uint8_t>(), c.dec_offs.as<uint32_t>(), d_cls);
+                                                                                c.dec_syms.as<uint8_t>(), c.dec_offs.as<uint32_t>(), d_cls, nullptr);
     decode_kernel<L, 2><<<n_chunks, DEC_THREADS, sizeof(DecodeSmem), stream>>>(fp, d_chunks, d_st, d_index, index_len, static_cast<L*>(d_out), out_len, c.d_binoms,
-                                                                                c.dec_syms.as<uint8_t>(), c.dec_offs.as<uint32_t>(), d_cls);
+                                                                                c.dec_syms.as<uint8_t>(), c.dec_offs.as<uint32_t>(), d_cls, nullptr);
     return 0;
   });
   profiler().end(stream);
@@ -563,6 +569,42 @@ static PcoB200Error decompress_core(const void* compressed, size_t compressed_le
   return e;
 }
 
+// ---- stream-ordered decompress (pco_b200_decompress_async) ---------------------------------------------------------------------------
+// The caller's workspace, from a 256-byte aligned base: gate | binomials | statuses | class bytes | the general pair's symbol rows |
+// its section starts.  The rows are sized from n_total (the kernels' out_len), as scratch_rows_total does for a 64-bit chunk count.
+struct AsyncLayout {
+  size_t gate, binoms, statuses, cls, syms, offs, total;
+};
+static AsyncLayout async_layout(uint64_t n_total, uint64_t n_chunks) {
+  auto up = [](uint64_t x) { return (x + 255) & ~uint64_t(255); };
+  const uint64_t rows = uint64_t(MAX_VARS) * (n_total / BATCH_N + n_chunks + 1);
+  AsyncLayout l;
+  uint64_t o = 0;
+  l.gate = o; o += up(sizeof(AsyncGate));
+  l.binoms = o; o += up(sizeof(Binoms));
+  l.statuses = o; o += up(n_chunks * sizeof(uint32_t));
+  l.cls = o; o += up(n_chunks);
+  l.syms = o; o += up(rows * BATCH_N + 64);
+  l.offs = o; o += up(rows * sizeof(uint32_t) + 64);
+  l.total = o + 256;  // room to align the caller's pointer
+  return l;
+}
+
+// The thread context's one-time set-up (device, binomials, kernel attributes) runs synchronous CUDA calls, which a stream capture
+// refuses: during a capture it has to have happened already.
+static PcoB200Error async_setup(Context& c, cudaStream_t stream) {
+  int cur = -1;
+  const bool ready = c.initialized && c.device_ok && c.attrs_set && cudaGetDevice(&cur) == cudaSuccess && cur == c.device;
+  if (!ready) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(stream, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone)
+      return fail(PCO_B200_CUDA, "the first pco_b200_decompress_async on a thread and device cannot be captured: call pco_b200_decompress_async_prepare before capturing");
+    cudaGetLastError();
+  }
+  if (PcoB200Error e = ensure_device(c)) return e;
+  return set_decode_attrs(c);
+}
+
 }  // namespace pcob200
 
 using namespace pcob200;
@@ -615,6 +657,63 @@ PcoB200Error pco_b200_decompress_ex(const void* compressed, size_t compressed_le
     progress->n_processed = size_t(std::min<uint64_t>(oc.n_total, dst_len));
     progress->finished = (oc.terminated && oc.n_total <= dst_len) ? 1 : 0;
   }
+  return PCO_B200_OK;
+}
+
+size_t pco_b200_decompress_async_workspace_size(size_t n_total, size_t n_chunks, unsigned char dtype) {
+  if (!nt_valid(dtype)) return 0;
+  return size_t(async_layout(n_total, n_chunks).total);
+}
+
+PcoB200Error pco_b200_decompress_async_prepare(unsigned char dtype) {
+  if (!nt_valid(dtype)) return fail(PCO_B200_INVALID_TYPE, "unknown number type byte: " + std::to_string(dtype));
+  return async_setup(ctx(), nullptr);
+}
+
+// Six launches on `cuda_stream` and nothing else: async_validate_kernel, fused_narrow_kernel, symwalk_kernel, decode_kernel<L, 1>,
+// decode_kernel<L, 2>, async_outcome_kernel.  The general pair runs whatever the fused kernel left, since the host does not look: the
+// chunks the fused kernel finished leave its CTAs at once through their class bytes.
+PcoB200Error pco_b200_decompress_async(const void* d_src, size_t src_len, unsigned char dtype, const void* d_index, size_t index_len, size_t n_chunks,
+                                       size_t n_total, void* d_dst, size_t dst_len, void* d_workspace, size_t workspace_len, PcoB200AsyncResult* d_result,
+                                       void* cuda_stream) {
+  if (!nt_valid(dtype)) return fail(PCO_B200_INVALID_TYPE, "unknown number type byte: " + std::to_string(dtype));
+  if (!d_src || !d_index || !d_dst || !d_workspace || !d_result) return fail(PCO_B200_INVALID_ARGUMENT, "null pointer");
+  if (n_chunks == 0 || n_chunks > 0x7fffffffull) return fail(PCO_B200_INVALID_ARGUMENT, "n_chunks must be 1..2^31 - 1");
+  if (dst_len < n_total) return fail(PCO_B200_INVALID_ARGUMENT, "dst holds " + std::to_string(dst_len) + " numbers, the file " + std::to_string(n_total));
+  if (index_len < sizeof(IndexHeader) || (index_len - sizeof(IndexHeader)) / sizeof(IndexChunk) < n_chunks)
+    return fail(PCO_B200_INVALID_ARGUMENT, "side index is shorter than its chunk table");
+  if (reinterpret_cast<uintptr_t>(d_index) & 7) return fail(PCO_B200_INVALID_ARGUMENT, "side index must be 8-byte aligned");
+  const AsyncLayout lay = async_layout(n_total, n_chunks);
+  if (workspace_len < lay.total)
+    return fail(PCO_B200_INVALID_ARGUMENT, "workspace holds " + std::to_string(workspace_len) + " bytes, the call needs " + std::to_string(lay.total));
+  Context& c = ctx();
+  cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+  if (PcoB200Error e = async_setup(c, stream)) return e;
+  uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(d_workspace) + 255) & ~uintptr_t(255));
+  AsyncGate* gate = reinterpret_cast<AsyncGate*>(ws + lay.gate);
+  const uint32_t* gate_words = reinterpret_cast<const uint32_t*>(gate);
+  Binoms* binoms = reinterpret_cast<Binoms*>(ws + lay.binoms);
+  uint32_t* d_st = reinterpret_cast<uint32_t*>(ws + lay.statuses);
+  uint8_t* d_cls = ws + lay.cls;
+  uint8_t* d_syms = ws + lay.syms;
+  uint32_t* d_offs = reinterpret_cast<uint32_t*>(ws + lay.offs);
+  const uint8_t* d_idx = static_cast<const uint8_t*>(d_index);
+  const IndexChunk* d_chunks = reinterpret_cast<const IndexChunk*>(d_idx + sizeof(IndexHeader));  // chunks_offset is checked on the device
+  const uint32_t grid = uint32_t(n_chunks);
+  // uniform_type and format_major come from the gate; the kernels write no number at or beyond n_total
+  FileParams fp{d_src, uint64_t(src_len), dtype, 0, 4};
+  async_validate_kernel<<<1, 32, 0, stream>>>(static_cast<const uint8_t*>(d_src), src_len, dtype, d_idx, index_len, n_chunks, n_total, gate, binoms, d_result);
+  dispatch_latent(dtype, [&](auto tag) {
+    using L = decltype(tag);
+    L* out = static_cast<L*>(d_dst);
+    fused_narrow_kernel<L><<<grid, FZ_THREADS, sizeof(FusedSmem), stream>>>(fp, d_chunks, d_idx, index_len, d_st, d_cls, out, n_total, gate_words);
+    symwalk_kernel<<<grid, SW_THREADS, sizeof(SymWalkSmem), stream>>>(fp, d_chunks, d_idx, index_len, n_total, d_syms, d_offs, d_cls, nullptr, 1, gate_words);
+    decode_kernel<L, 1><<<grid, DEC_THREADS, sizeof(DecodeSmem), stream>>>(fp, d_chunks, d_st, d_idx, index_len, out, n_total, binoms, d_syms, d_offs, d_cls, gate_words);
+    decode_kernel<L, 2><<<grid, DEC_THREADS, sizeof(DecodeSmem), stream>>>(fp, d_chunks, d_st, d_idx, index_len, out, n_total, binoms, d_syms, d_offs, d_cls, gate_words);
+    return 0;
+  });
+  async_outcome_kernel<<<1, OUTCOME_THREADS, 0, stream>>>(gate_words, d_st, d_cls, grid, d_result);
+  PCOB_CUDA_TRY(cudaGetLastError());
   return PCO_B200_OK;
 }
 
